@@ -38,6 +38,13 @@ B=32, get_loss = 2 FPS + 3 Chamfer terms + one collective; forward + backward ca
 dist.GraphedLoss, the eager autograd call timed beside it as `eager`).
 `--impl reference` times the CPU expression alone (the reference has no CPU kernel of its own;
 metrics/CD/chamfer_python.py is its pure-torch restatement) on the same config/metric, full B=32 per step.
+`--steps K` is the number of timed steps of the headline in all: the `--repeats` blocks share them (default 140 = 7
+blocks of 20).  The side measurements size their own loops from K: the forward-only roofline timing max(10, K) launches,
+e2e K calls one at a time, 3 blocks of K overlapped steps and K loss-readback calls, fresh buffers max(K, 24) calls,
+serial max(3, K // 4) calls.
+`--dump-outputs DIR` writes what the timed step returned in its last timed run (rank 0's share) as DIR/<name>.npy,
+float32 / float64 (indices as float64, exact); the inputs are seeded, so two builds can be compared output for output.
+Inside the tree, `bench_outputs/` is the git-ignored place for them.
 """
 import argparse
 import importlib.util
@@ -52,7 +59,9 @@ import time
 ROOT = osp.dirname(osp.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: nothing is written next to the sources
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 C1 = dict(B=32, N=2048, M=16384)
@@ -175,6 +184,20 @@ def timed_pipelined(fn, iters, warmup, flush):
     return [a.elapsed_time(b) for a, b in evs]
 
 
+def dump_outputs(out_dir, arrays):
+    """{name: tensor} -> out_dir/<name>.npy, floating point kept as is (float32 / float64), integers as float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        np.save(osp.join(out_dir, name + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
+
+
+def block_sizes(steps, repeats):
+    """`steps` timed steps split into at most `repeats` blocks of near-equal length."""
+    n = max(1, min(repeats, steps))
+    return [steps // n + (1 if i < steps % n else 0) for i in range(n)]
+
+
 def max_over_ranks(x, dev, world, dist):
     t = torch.tensor([x], device=dev, dtype=torch.float64)
     if world > 1:
@@ -251,12 +274,17 @@ def run_ours(args):
         flush_buf.zero_()
 
     launches_per_step = [0]
+    out_names = ("dist1", "dist2", "idx1", "idx2", "gradxyz1", "gradxyz2", "loss_sums")
     if reduce_mode in ("none (1 GPU)", "peer"):
         stepper = ps.ChamferStep(B, N, M, dev, comm=comm)
         stepper.prepare(x1, x2, gd1, gd2)  # capture + instantiate outside any loop
 
         def step():
             stepper(x1, x2, gd1, gd2)  # ONE cudaGraphLaunch
+
+        def outputs():
+            s = stepper
+            return dict(zip(out_names, (s.dist1, s.dist2, s.idx1, s.idx2, s.gradxyz1, s.gradxyz2, s.sums_global)))
     elif reduce_mode == "nccl_graph":
         # the same five kernels + ncclAllReduce captured into one torch CUDA graph
         fwd_out = (torch.empty(B, N, device=dev), torch.empty(B, M, device=dev),
@@ -286,6 +314,9 @@ def run_ours(args):
 
         def step():
             graph.replay()
+
+        def outputs():
+            return dict(zip(out_names, fwd_out + bwd_out + (gsum,)))
     else:  # "pipelined" / "inline": round 1's eager issue, kept for A/B
         reducer = PipelinedSums()
         fwd_out = (torch.empty(B, N, device=dev), torch.empty(B, M, device=dev),
@@ -304,6 +335,9 @@ def run_ours(args):
             if reduce_mode == "pipelined":
                 reducer.submit(vec)
 
+        def outputs():
+            return dict(zip(out_names, fwd_out + bwd_out + (sum_bufs[(step_no[0] - 1) & 1],)))
+
     # ---- warm-up, fp32 peak, forward-only timing for the roofline ------------------------------
     for _ in range(max(args.warmup, 3)):
         step()
@@ -319,7 +353,7 @@ def run_ours(args):
     sampler = ClockSampler(local_rank)
     sampler.start()
     blocks, host_ms_blocks, launches = [], [], 0
-    for rep in range(max(1, args.repeats)):
+    for nsteps in block_sizes(args.steps, args.repeats):
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
@@ -329,7 +363,7 @@ def run_ours(args):
         L.launch_count(reset=True)
         evs = []
         t_host0 = time.perf_counter()
-        for _ in range(args.steps):
+        for _ in range(nsteps):
             flush()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
@@ -338,13 +372,15 @@ def run_ours(args):
             evs.append((e0, e1))
         t_issue = time.perf_counter() - t_host0
         torch.cuda.synchronize()
-        launches = L.launch_count(reset=True) + launches_per_step[0] * args.steps
+        launches = L.launch_count(reset=True) + launches_per_step[0] * nsteps
         if world > 1:
             dist.barrier()
         total_ms = sum(a.elapsed_time(b) for a, b in evs)
-        blocks.append(max_over_ranks(total_ms, dev, world, dist) / args.steps)
-        host_ms_blocks.append(t_issue * 1e3 / args.steps)
+        blocks.append(max_over_ranks(total_ms, dev, world, dist) / nsteps)
+        host_ms_blocks.append(t_issue * 1e3 / nsteps)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs())
     ms_per_step = statistics.median(blocks)
     pairs_per_step = 2.0 * B * N * M
     value = pairs_per_step * world / (ms_per_step * 1e-3) / 1e9  # Gpair/s, whole job
@@ -499,8 +535,8 @@ def run_ours(args):
                                   "nccl_graph": "every step: ncclAllReduce of the 6 loss sums captured inside the step's CUDA graph",
                                   "pipelined": "c10d all-reduce issued asynchronously and joined one step later (round-1 path)",
                                   "inline": "c10d all-reduce in line between forward and backward (round-1 A/B path)"}[reduce_mode],
-                   "timing": f"median of {len(blocks)} blocks of {args.steps} steps; each block: barrier + synchronize, 3 untimed lockstep steps, "
-                             f"{args.steps} steps timed with CUDA events, max over ranks",
+                   "timing": f"{args.steps} timed steps in {len(blocks)} blocks, median block; each block: barrier + synchronize, 3 untimed "
+                             "lockstep steps, then its steps timed with CUDA events, max over ranks",
                    "parallelism": f"batch-sharded x{world}"},
         "blocks_ms_per_step": [round(b, 4) for b in blocks],
         "spread": {"min": round(min(blocks), 4), "max": round(max(blocks), 4), "median": round(ms_per_step, 4)},
@@ -593,14 +629,14 @@ def run_c4loss(args, ps, dist, dev, rank, world, comm, reduce_mode):
         for _ in range(max(args.warmup, 3)):
             fn()
         blocks = []
-        for rep in range(max(1, args.repeats)):
+        for nsteps in block_sizes(args.steps, args.repeats):
             torch.cuda.synchronize()
             if world > 1:
                 dist.barrier()
             fn()
             torch.cuda.synchronize()
             evs = []
-            for _ in range(args.steps):
+            for _ in range(nsteps):
                 flush_buf.zero_()
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 e0.record()
@@ -608,11 +644,14 @@ def run_c4loss(args, ps, dist, dev, rank, world, comm, reduce_mode):
                 e1.record()
                 evs.append((e0, e1))
             torch.cuda.synchronize()
-            blocks.append(max_over_ranks(sum(a.elapsed_time(b) for a, b in evs), dev, world, dist) / args.steps)
+            blocks.append(max_over_ranks(sum(a.elapsed_time(b) for a, b in evs), dev, world, dist) / nsteps)
         return blocks
 
     eager_blocks = timed_blocks(step)
     blocks = timed_blocks(step_graphed)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": graphed.loss.reshape(1), "loss_terms": torch.stack(graphed.terms),
+                                         **{f"grad_pred{i}": g for i, g in enumerate(graphed.grads)}})
     ms, eager_ms = statistics.median(blocks), statistics.median(eager_blocks)
     pairs = 2.0 * Btot * (512 * 512 + 2048 * 2048 + 16384 * 16384)
     if rank == 0:
@@ -918,10 +957,10 @@ def main():
     claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=140, help="timed steps of the headline in all")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
-    ap.add_argument("--repeats", type=int, default=7, help="how many times the K-step block is timed (median reported)")
+    ap.add_argument("--repeats", type=int, default=7, help="how many blocks the K timed steps are split into (median block reported)")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"])
     ap.add_argument("--workload", default="c5", choices=["c1", "c5", "c4loss"], help="--scaling strong: which fixed-size workload to split")
     ap.add_argument("--e2e-depth", type=int, default=4, help="steps in flight in the e2e loop (1-4; 1 = one call at a time)")
@@ -933,7 +972,12 @@ def main():
     ap.add_argument("--no-ref-cuda", action="store_true", help="skip timing the reference's CUDA kernels (oracle/_ref)")
     ap.add_argument("--quick", action="store_true", help="headline + e2e only")
     ap.add_argument("--ref-clouds", type=int, default=0, help="--impl reference: clouds per step (0 = the full B=32)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (in the tree: bench_outputs/)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the CUDA path's outputs (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,8 +1,8 @@
 """Generate tests/golden/*.npz from the REFERENCE's own CUDA ops (oracle/_ref) on a B200.
 
-Run on the GPU box (no /root/reference there; only the prebuilt oracle/_ref/*.so travel):
-    gpurun -- 'python tests/golden/make_golden.py gpurun_out/golden'
-then copy gpurun_out/golden/*.npz into tests/golden/ and commit them.
+Needs oracle/_ref/*.so (oracle/build_ref.py builds them from a checkout of the reference) and a B200:
+    python tests/golden/make_golden.py OUT_DIR
+then copy OUT_DIR/*.npz into tests/golden/ and commit them.
 
 Every case stores its seeded inputs next to the reference outputs, so the fixtures are
 self-contained.  kNN has no reference kernel: its golden output is the reference's torch
@@ -147,8 +147,12 @@ def main(out_dir):
         cases[f"{name}.k"] = np.int32(k)
         cases[f"{name}.include_self"] = np.int32(inc)
         if name in ("small", "dups"):
-            cases[f"{name}.dist"] = dist.cpu().numpy()
-            cases[f"{name}.dot"] = torch.matmul(Q, X.permute(0, 2, 1)).cpu().numpy()
+            rows = slice(None)
+            if name == "dups":  # a seeded sample of 8 query rows keeps the file small
+                cases[f"{name}.rows"] = np.sort(np.random.default_rng(0).choice(S, 8, replace=False)).astype(np.int32)
+                rows = torch.as_tensor(cases[f"{name}.rows"], dtype=torch.long, device=dev)
+            cases[f"{name}.dist"] = dist[:, rows].cpu().numpy()
+            cases[f"{name}.dot"] = torch.matmul(Q, X.permute(0, 2, 1))[:, rows].cpu().numpy()
             cases[f"{name}.qq"] = torch.sum(Q ** 2, -1).cpu().numpy()
     np.savez_compressed(osp.join(out_dir, "knn.npz"), **cases)
     print("golden vectors written to", out_dir, "| torch", torch.__version__, "| gpu", torch.cuda.get_device_name(0))

@@ -1,9 +1,9 @@
 """Golden vectors for the SURVEY 8(f) "next" rows, generated on a B200 from the reference's own
 CUDA ops (oracle/_ref) combined by the reference's torch expressions (restated in oracle/oracle.py
 with file:line citations; tests/test_reference_python.py checks those restatements against the
-reference's Python, imported from /root/reference, wherever that tree is present).
+reference's Python wherever a checkout of it is present).
 
-    gpurun -- 'python tests/golden/make_golden_next.py gpurun_out/golden'
+    python tests/golden/make_golden_next.py OUT_DIR
 
   next.npz            committed fixture: sample_and_group_knn, EdgeConv edge features (C=3 and
                       feature space), calc_cd / fscore / calc_dcd
@@ -67,7 +67,9 @@ def main(out_dir):
         X = x.to(dev)
         feat, idx = O.torch_edge_features(X, k)
         torch.cuda.synchronize()
-        cases.update({f"{name}.x": x.numpy(), f"{name}.k": np.int32(k), f"{name}.idx": idx.int().cpu().numpy()})
+        cases.update({f"{name}.k": np.int32(k), f"{name}.idx": idx.int().cpu().numpy()})
+        if name != "edge256":  # 0.5 MB of noise: tests/conftest.py redraws it from this seed sequence
+            cases[f"{name}.x"] = x.numpy()
         if N * k * C <= 200000:
             cases[f"{name}.feat"] = feat.cpu().numpy()
         xt = X.transpose(2, 1).contiguous()

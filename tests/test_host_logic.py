@@ -6,7 +6,7 @@ import sys
 import pytest
 import torch
 
-from conftest import ROOT
+from conftest import REFERENCE, ROOT
 import svdformer_pointsea_b200 as ps
 from svdformer_pointsea_b200 import _lib as L
 
@@ -61,10 +61,11 @@ def test_missing_library_fails_loudly(monkeypatch, tmp_path):
 
 def test_reference_loss_utils_imports_unchanged_when_reference_present():
     """utils/loss_utils.py:3-6 imports models.model_utils (which needs our six pointnet2 names) and
-    metrics.CD.* — with the drop-in ahead on sys.path the import works without building anything."""
-    ref = "/root/reference"
+    metrics.CD.* — with the drop-in ahead on sys.path the import works without building anything.
+    Runs where a checkout of the reference (not part of this repository) is present."""
+    ref = REFERENCE
     if not osp.isdir(ref):
-        pytest.skip("reference tree not present on this box")
+        pytest.skip(f"needs a checkout of the reference at {ref} (or set POINTSEA_REFERENCE)")
     ps.install_dropin()
     added = ref not in sys.path
     if added:

@@ -77,11 +77,12 @@ def test_knn_matches_torch_cuda_golden():
 
 def test_knn_distance_arithmetic_matches_torch_cuda_bits():
     """The stored (S,N) distance rows pin the fp32 arithmetic: dot = fma(z,z',fma(y,y',x*x')),
-    |p|^2 = (x^2 + z^2) + y^2, dist = ((-2*dot) + |q|^2) + |p|^2."""
+    |p|^2 = (x^2 + z^2) + y^2, dist = ((-2*dot) + |q|^2) + |p|^2.  'dups' stores a seeded sample of its rows."""
     z = load_golden("knn")
     f = np.float32
     for name in ("small", "dups"):
-        q, p, dist = z[f"{name}.new_xyz"], z[f"{name}.xyz"], z[f"{name}.dist"]
+        rows = z[f"{name}.rows"] if f"{name}.rows" in z.files else slice(None)
+        q, p, dist = z[f"{name}.new_xyz"][:, rows], z[f"{name}.xyz"], z[f"{name}.dist"]
 
         def ss(v):
             a, b, c = [(v[..., i] * v[..., i]).astype(f) for i in range(3)]

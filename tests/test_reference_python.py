@@ -1,8 +1,8 @@
 """Checks the oracle's torch restatements of the reference's PYTHON call sites against the reference's
-own functions, imported from /root/reference with its CUDA ops replaced by the CPU oracle.  Runs only where
-the reference tree exists (this container); the GPU box has no /root/reference and skips."""
+own functions, imported from a checkout of the reference with its CUDA ops replaced by the CPU oracle.
+The reference is not part of this repository: these tests run where a checkout of it is present
+(POINTSEA_REFERENCE, else BASELINE.json's reference_path) and skip otherwise."""
 import importlib
-import os
 import os.path as osp
 import sys
 import types
@@ -11,10 +11,12 @@ import numpy as np
 import pytest
 import torch
 
+from conftest import REFERENCE
 from oracle import oracle as O
 
-REF = os.environ.get("POINTSEA_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not osp.isdir(osp.join(REF, "models")), reason="reference tree not present")
+REF = REFERENCE
+pytestmark = pytest.mark.skipif(not osp.isdir(osp.join(REF, "models")),
+                                reason=f"needs a checkout of the reference at {REF} (or set POINTSEA_REFERENCE)")
 
 
 class _OracleChamfer(torch.nn.Module):

@@ -1,4 +1,4 @@
-import sys; sys.path.insert(0,'/root/repo')
+import os.path as osp, sys; sys.path.insert(0, osp.dirname(osp.dirname(osp.abspath(__file__))))
 import torch, time
 import svdformer_pointsea_b200 as ps
 g=torch.Generator().manual_seed(0)
