@@ -293,6 +293,20 @@ int ps_index_points_bwd(const float* grad_out, const int* idx, float* grad_point
 int ps_chamfer_metrics(const float* dist1, const float* dist2, const int* idx1, const int* idx2, float* out8,
                        int B, int n1, int n2, float fscore_threshold, float dcd_alpha, float dcd_n_lambda,
                        float dcd_frac1, float dcd_frac2, int dev, void* stream);
+/* Backward of ps_chamfer_metrics' differentiable outputs (what makes calc_cd / calc_dcd training losses): per-cloud
+ * upstream gradients -> per-point gradients of the distances, which ps_chamfer_bwd turns into point gradients.
+ * terms: bitmask of the per-cloud upstream gradients present in gcoef5 (B,5) =
+ *   bit0 mean sqrt d1, bit1 mean sqrt d2, bit2 mean d1, bit3 mean d2, bit4 dcd; other bits are rejected.
+ *   A clear bit contributes nothing (gcoef5 may be NULL when terms == 0); bit4 needs idx1 and idx2.
+ * graw1 (B,n1) / graw2 (B,n2): upstream gradients of the raw dist outputs, or NULL.
+ * graddist1 (B,n1), graddist2 (B,n2): OVERWRITTEN.  Other arguments as ps_chamfer_metrics.
+ *   graddist1[j] = graw1[j] + g0/n1 / (2 sqrt d1[j]) + g2/n1 + g4*0.5/n1 * alpha * exp(-alpha d1[j]) * w1[j]
+ *   (w1 = calc_dcd's weight of the hit count of idx1[j], detached); side 2 likewise with bits 1, 3, 4 and dcd_frac2.
+ *   torch's formulas, unclamped: a present sqrt term at d = 0 yields inf, as the reference's does. */
+int ps_chamfer_metrics_bwd(const float* dist1, const float* dist2, const int* idx1, const int* idx2,
+                           const float* gcoef5, unsigned terms, const float* graw1, const float* graw2,
+                           float* graddist1, float* graddist2, int B, int n1, int n2, float dcd_alpha,
+                           float dcd_n_lambda, float dcd_frac1, float dcd_frac2, int dev, void* stream);
 
 /* ---- measurement helpers (bench.py) ------------------------------------------------------
  * Runs an FFMA2-only kernel on `dev` and returns the best-of-`reps` fp32 TFLOP/s: the live

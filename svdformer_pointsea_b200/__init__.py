@@ -21,7 +21,7 @@ from .pointnet2_utils import (  # noqa: F401
 from .model_ops import (  # noqa: F401
     query_knn_point, index_points, group_local, edge_features, EdgeConv, sample_and_group_knn, knn_self, patch_model_utils,
 )
-from .metrics import calc_cd, calc_dcd, fscore, chamfer_metrics_raw, patch_loss_utils  # noqa: F401
+from .metrics import calc_cd, calc_dcd, fscore, chamfer_metrics_raw, chamfer_metrics_grad_raw, patch_loss_utils  # noqa: F401
 from .dropin import install_dropin, DROPIN_PATH  # noqa: F401
 
 __version__ = "0.1.0"
