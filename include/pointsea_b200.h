@@ -308,6 +308,20 @@ int ps_chamfer_metrics_bwd(const float* dist1, const float* dist2, const int* id
                            float* graddist1, float* graddist2, int B, int n1, int n2, float dcd_alpha,
                            float dcd_n_lambda, float dcd_frac1, float dcd_frac2, int dev, void* stream);
 
+/* ---- scatter-max (PointSea's depth-map renderer) ------------------------------------------
+ * torch_scatter.scatter(src, index, dim, out, dim_size, reduce="max") as models_PointSea/mv_utils_zs.py:130 calls it.
+ * src (outer, E, inner) f32, index (outer, E, inner) i64 (already broadcast to src's shape), out (outer, D, inner) f32.
+ * fresh != 0: out is initialised here and positions that receive nothing become 0 (torch_scatter without `out=`;
+ *   as there, a max of exactly -FLT_MAX also reads 0);
+ * fresh == 0: out's current values take part in the max (torch_scatter with `out=`), updated in place; a NaN there
+ *   is kept (a negative NaN pattern becomes the canonical positive one once a src element reaches it).
+ * argmax (outer, D, inner) i64 or NULL: position along E of the lowest-index src element equal to the result (NaN
+ *   matching NaN), E if none.
+ * Index values outside [0, D) are skipped.  NaN propagates (canonical positive NaN); +0 is larger than -0.  The result
+ * does not depend on the order of the updates. */
+int ps_scatter_max(const float* src, const long long* index, float* out, long long* argmax, long long outer,
+                   long long E, long long inner, long long D, int fresh, int dev, void* stream);
+
 /* ---- measurement helpers (bench.py) ------------------------------------------------------
  * Runs an FFMA2-only kernel on `dev` and returns the best-of-`reps` fp32 TFLOP/s: the live
  * roofline denominator for the Chamfer kernel (MEASURED_PEAKS.json has no fp32 figure).

@@ -9,7 +9,8 @@ Public surface = the reference's op boundary (SURVEY.md 8b):
     calc_cd, calc_dcd, fscore                                 (utils/loss_utils.py, metrics/CD/fscore.py)
 `install_dropin()` makes `import metrics.CD.chamfer3D.dist_chamfer_3D` and
 `import pointnet2_ops.pointnet2_utils` resolve to this package so the reference's models and
-losses run unchanged.
+losses run unchanged, and `import torch_scatter` too where no torch_scatter is installed
+(svdformer_pointsea_b200.scatter: PointSea's scatter-max).
 """
 from ._lib import PointSeaError, LIB_PATH, load as load_library  # noqa: F401
 from .chamfer import chamfer_3DDist, chamfer_3DFunction, chamfer_forward, chamfer_backward, chamfer_sums, chamfer_host, chamfer_host_async, HostStep, chamfer_host_step, ChamferStep  # noqa: F401
@@ -22,6 +23,6 @@ from .model_ops import (  # noqa: F401
     query_knn_point, index_points, group_local, edge_features, EdgeConv, sample_and_group_knn, knn_self, patch_model_utils,
 )
 from .metrics import calc_cd, calc_dcd, fscore, chamfer_metrics_raw, chamfer_metrics_grad_raw, patch_loss_utils  # noqa: F401
-from .dropin import install_dropin, DROPIN_PATH  # noqa: F401
+from .dropin import install_dropin, DROPIN_PATH, DROPIN_FALLBACK_PATH  # noqa: F401
 
 __version__ = "0.1.0"

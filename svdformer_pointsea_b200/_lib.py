@@ -62,6 +62,8 @@ _SIGNATURES = {
                            _c_float, _c_int, _P],
     "ps_chamfer_metrics_bwd": [_P, _P, _P, _P, _P, ctypes.c_uint, _P, _P, _P, _P, _c_int, _c_int, _c_int, _c_float,
                                _c_float, _c_float, _c_float, _c_int, _P],
+    "ps_scatter_max": [_P, _P, _P, _P, ctypes.c_longlong, ctypes.c_longlong, ctypes.c_longlong, ctypes.c_longlong,
+                       _c_int, _c_int, _P],
     "ps_three_nn": [_P, _P, _P, _P, _c_int, _c_int, _c_int, _c_int, _P],
     "ps_three_interpolate_fwd": [_P, _P, _P, _P, _c_int, _c_int, _c_int, _c_int, _c_int, _P],
     "ps_three_interpolate_bwd": [_P, _P, _P, _P, _c_int, _c_int, _c_int, _c_int, _c_int, _P],

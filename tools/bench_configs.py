@@ -8,10 +8,13 @@ C4  full SVDFormer PCN forward + Chamfer loss, random-init weights (seed 1), B=3
     The reference tree is not part of this repository: stage it (git-ignored) with
         cp -r /root/reference baseline/_ref/reference
     before `gpurun`.  Each arm runs in its own process (they bind the same module names).
+    PointSea's renderer imports torch_scatter (models_PointSea/mv_utils_zs.py:1,130).  --torch-scatter stub (default)
+    stands it in by Tensor.scatter_reduce_ in both arms; --torch-scatter dropin makes the "ours" arm import it through
+    install_dropin()'s fallback path (svdformer_pointsea_b200.scatter, the sm_100a scatter-max) instead.
 C5  stress: Chamfer fwd+bwd and FPS 131072 -> 16384 on B=8 clouds of 131072 points (split over the
     ranks), parity against the reference kernels on rank 0, NCCL all-reduce of the loss sums.
 
-usage:  python tools/bench_configs.py c4 [--arm ours|ref|both] [--iters 5]
+usage:  python tools/bench_configs.py c4 [--arm ours|ref|both] [--iters 5] [--model pointsea --torch-scatter stub|dropin]
         python tools/bench_configs.py c5
         torchrun --nproc-per-node G tools/bench_configs.py c5      (sharded)
 """
@@ -82,7 +85,7 @@ def install_torch_scatter_stub():
     sys.modules["torch_scatter"] = m
 
 
-def c4_arm(arm, iters, knn, batch=32, model_name="svdformer", loss_name="get_loss"):
+def c4_arm(arm, iters, knn, batch=32, model_name="svdformer", loss_name="get_loss", torch_scatter="stub"):
     rank, world, dev = dist_setup()
     if not osp.isdir(REF_TREE):
         print(json.dumps({"config": "C4", "arm": arm, "unavailable": f"{REF_TREE} not staged"}))
@@ -113,7 +116,8 @@ def c4_arm(arm, iters, knn, batch=32, model_name="svdformer", loss_name="get_los
         import pointnet2_ops  # noqa: F401  (binds the reference wrappers to the reference kernels)
         pointnet2_ops._ext = ref_pn
     from types import SimpleNamespace as NS
-    install_torch_scatter_stub()
+    if arm != "ours" or torch_scatter == "stub":
+        install_torch_scatter_stub()
     # no network on the box: PointSea asks torchvision for ImageNet weights (PointSea.py:40); random init instead
     import torchvision.models as tvm
     _resnet18 = tvm.resnet18
@@ -188,6 +192,8 @@ def c4_arm(arm, iters, knn, batch=32, model_name="svdformer", loss_name="get_los
            "ms_loss_min": round(min(tl), 3), "loss": float(out["loss"]), "losses": [float(x) for x in out["losses"]],
            "loss_hex": float(out["loss"]).hex(), "losses_hex": [float(x).hex() for x in out["losses"]],
            "model": model_name, "loss_fn": loss_name, "batch": batch}
+    if "torch_scatter" in sys.modules:  # where PointSea's scatter came from: the stub (no file) or a package
+        res["torch_scatter"] = getattr(sys.modules["torch_scatter"], "__file__", None) or "stub"
     if rank == 0:
         print(json.dumps(res))
     if world > 1:
@@ -199,11 +205,11 @@ def c4_arm(arm, iters, knn, batch=32, model_name="svdformer", loss_name="get_los
 def c4(args):
     arms = ["ours", "ref"] if args.arm == "both" else [args.arm]
     if args.arm != "both":
-        return c4_arm(args.arm, args.iters, args.knn, args.batch, args.model, args.loss)
+        return c4_arm(args.arm, args.iters, args.knn, args.batch, args.model, args.loss, args.torch_scatter)
     lines = []
     for arm, knn in (("ours", "torch"), ("ours", "ours"), ("ours", "all"), ("ref", "torch")):
         p = subprocess.run([sys.executable, __file__, "c4", "--arm", arm, "--iters", str(args.iters), "--knn", knn, "--batch", str(args.batch),
-                            "--model", args.model, "--loss", args.loss],
+                            "--model", args.model, "--loss", args.loss, "--torch-scatter", args.torch_scatter],
                            capture_output=True, text=True)
         last = [ln for ln in p.stdout.strip().splitlines() if ln.startswith("{")]
         if not last:
@@ -277,5 +283,7 @@ if __name__ == "__main__":
     ap.add_argument("--batch", type=int, default=32, help="c4: total clouds")
     ap.add_argument("--model", default="svdformer", choices=["svdformer", "pointsea"])
     ap.add_argument("--loss", default="get_loss", choices=["get_loss", "get_loss_PM"])
+    ap.add_argument("--torch-scatter", default="stub", choices=["stub", "dropin"],
+                    help="c4 pointsea: arm ours imports torch_scatter from the drop-in instead of the stand-in")
     a = ap.parse_args()
     {"c4": c4, "c5": c5}[a.config](a)
