@@ -77,6 +77,27 @@ int ps_chamfer_sums(const float* dist1, const float* dist2, double* out6, long l
 int ps_chamfer_fwd_sums(const float* xyz1, const float* xyz2, float* dist1, float* dist2, int* idx1, int* idx2,
                         double* sums6, int B, int N, int M, int dev, void* stream);
 
+/* ---- Chamfer training losses (utils/loss_utils.py:10-31) as one forward and one backward ----------------------
+ * n1 = B*N and n2 = B*M are the element counts torch.mean divides by.  Other kind values are rejected. */
+#define PS_LOSS_CD 0          /* chamfer:                  mean(d1) + mean(d2)               */
+#define PS_LOSS_CD_SQRT 1     /* chamfer_sqrt:             (mean(sqrt d1) + mean(sqrt d2)) / 2 */
+#define PS_LOSS_SINGLE 2      /* chamfer_single_side:      mean(d1)                          */
+#define PS_LOSS_SINGLE_SQRT 3 /* chamfer_single_side_sqrt: mean(sqrt d1)                     */
+/* ps_chamfer_fwd_sums (dist/idx and sums6, device, 6 doubles of scratch) followed by one single-thread launch that
+ * writes loss (device, 1 float): the sums combined in double and rounded once.  No host sync.  B = 0 gives NaN, as
+ * torch.mean of an empty tensor. */
+int ps_chamfer_loss_fwd(const float* xyz1, const float* xyz2, float* dist1, float* dist2, int* idx1, int* idx2,
+                        double* sums6, float* loss, int kind, int B, int N, int M, int dev, void* stream);
+/* Backward of ps_chamfer_loss_fwd: grad_loss (device, 1 float) is the upstream gradient of the loss.  Each point's
+ * distance gradient is derived from dist1/dist2 with torch's autograd of the reference expression (g*0.5 for the
+ * sqrt kinds' "/ 2", g * (1.0f/n), g / (2*sqrtf(d)) for the sqrt kinds: inf/NaN at d = 0 as in torch), then turned
+ * into point gradients with ps_chamfer_bwd's arithmetic.  gradxyz1 (B,N,3) / gradxyz2 (B,M,3): OVERWRITTEN (zero
+ * where no term reaches them); either may be NULL (its writes and scatters are skipped), not both.  Two launches:
+ * plain stores, then atomics; the second is skipped when no scattered term lands in a non-NULL buffer. */
+int ps_chamfer_loss_bwd(const float* xyz1, const float* xyz2, const float* dist1, const float* dist2, const int* idx1,
+                        const int* idx2, const float* grad_loss, float* gradxyz1, float* gradxyz2, int kind, int B,
+                        int N, int M, int dev, void* stream);
+
 /* ---- the single collective of the batch-sharded path (SURVEY 8e), over peer memory ---------------------------
  * The reference has no multi-process path (nn.DataParallel gathers on one GPU); its loss reductions
  * (utils/loss_utils.py:10-19,50-57) are what has to be summed across ranks.  A ps_comm is a set of per-rank

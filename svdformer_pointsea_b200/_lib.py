@@ -29,6 +29,8 @@ _SIGNATURES = {
     "ps_chamfer_host_wait": [ctypes.c_longlong, _c_int, _P, _c_int, _c_int],
     "ps_chamfer_host_step": [_P, _P, _P, _P, _P, _P, _P, _c_int, _c_int, _c_int, _c_int, _c_int, _P],
     "ps_chamfer_fwd_sums": [_P, _P, _P, _P, _P, _P, _P, _c_int, _c_int, _c_int, _c_int, _P],
+    "ps_chamfer_loss_fwd": [_P] * 8 + [_c_int, _c_int, _c_int, _c_int, _c_int, _P],
+    "ps_chamfer_loss_bwd": [_P] * 9 + [_c_int, _c_int, _c_int, _c_int, _c_int, _P],
     "ps_chamfer_step": [_P] * 13 + [_c_int, _c_int, _c_int, _c_int, _P],
     "ps_chamfer_step_prepare": [_P] * 13 + [_c_int, _c_int, _c_int, _c_int],
     "ps_chamfer_step_stats": [_c_int, ctypes.POINTER(ctypes.c_longlong), ctypes.POINTER(ctypes.c_longlong), ctypes.POINTER(ctypes.c_longlong)],

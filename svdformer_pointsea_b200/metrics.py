@@ -173,10 +173,18 @@ def calc_dcd(x, gt, alpha=1000, n_lambda=1, return_raw=False, non_reg=False):
     return res
 
 
-def patch_loss_utils(module):
+def patch_loss_utils(module, training=False):
     """Rebind calc_cd / calc_dcd / fscore inside an imported reference `utils.loss_utils` (evaluation loops call
-    them through that module: core/test_pcn.py:64, core/eval_55.py:74)."""
+    them through that module: core/test_pcn.py:64, core/eval_55.py:74).
+
+    training=True also rebinds chamfer / chamfer_sqrt / chamfer_single_side / chamfer_single_side_sqrt to the fused
+    ops of `losses`.  The reference's get_loss / get_loss_PM (:33-85) look these names up as module globals when they
+    run, so they then run on the fused ops unchanged."""
     module.calc_cd = calc_cd
     module.calc_dcd = calc_dcd
     module.fscore = fscore
+    if training:
+        from . import losses
+        for name in losses.TRAINING_LOSSES:
+            setattr(module, name, getattr(losses, name))
     return module

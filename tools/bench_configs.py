@@ -11,10 +11,13 @@ C4  full SVDFormer PCN forward + Chamfer loss, random-init weights (seed 1), B=3
     PointSea's renderer imports torch_scatter (models_PointSea/mv_utils_zs.py:1,130).  --torch-scatter stub (default)
     stands it in by Tensor.scatter_reduce_ in both arms; --torch-scatter dropin makes the "ours" arm import it through
     install_dropin()'s fallback path (svdformer_pointsea_b200.scatter, the sm_100a scatter-max) instead.
+    --loss-impl fused makes the "ours" arm call patch_loss_utils(utils.loss_utils, training=True), so get_loss /
+    get_loss_PM run their Chamfer terms on the fused ops; the result reports how many calls reached them.
 C5  stress: Chamfer fwd+bwd and FPS 131072 -> 16384 on B=8 clouds of 131072 points (split over the
     ranks), parity against the reference kernels on rank 0, NCCL all-reduce of the loss sums.
 
 usage:  python tools/bench_configs.py c4 [--arm ours|ref|both] [--iters 5] [--model pointsea --torch-scatter stub|dropin]
+                                           [--loss-impl composed|fused]
         python tools/bench_configs.py c5
         torchrun --nproc-per-node G tools/bench_configs.py c5      (sharded)
 """
@@ -85,7 +88,8 @@ def install_torch_scatter_stub():
     sys.modules["torch_scatter"] = m
 
 
-def c4_arm(arm, iters, knn, batch=32, model_name="svdformer", loss_name="get_loss", torch_scatter="stub"):
+def c4_arm(arm, iters, knn, batch=32, model_name="svdformer", loss_name="get_loss", torch_scatter="stub",
+           loss_impl="composed"):
     rank, world, dev = dist_setup()
     if not osp.isdir(REF_TREE):
         print(json.dumps({"config": "C4", "arm": arm, "unavailable": f"{REF_TREE} not staged"}))
@@ -137,6 +141,20 @@ def c4_arm(arm, iters, knn, batch=32, model_name="svdformer", loss_name="get_los
     else:
         from models.SVDFormer import Model  # after the patch: it does `from models.model_utils import *`
     import utils.loss_utils as lu
+    fused_calls = [0]
+    if loss_impl == "fused" and arm == "ours":
+        import svdformer_pointsea_b200 as ps
+        from svdformer_pointsea_b200 import losses
+        ps.patch_loss_utils(lu, training=True)
+
+        def counted(fn):
+            def call(*a, **k):
+                fused_calls[0] += 1
+                return fn(*a, **k)
+            return call
+        # count the calls that reach the rebound names, so a loss that does not look them up shows 0
+        for name in losses.TRAINING_LOSSES:
+            setattr(lu, name, counted(getattr(lu, name)))
     if loss_name == "get_loss_PM":
         def get_loss(preds, gt, sqrt=True):
             return lu.get_loss_PM(preds, partial, gt, sqrt=sqrt)
@@ -192,6 +210,9 @@ def c4_arm(arm, iters, knn, batch=32, model_name="svdformer", loss_name="get_los
            "ms_loss_min": round(min(tl), 3), "loss": float(out["loss"]), "losses": [float(x) for x in out["losses"]],
            "loss_hex": float(out["loss"]).hex(), "losses_hex": [float(x).hex() for x in out["losses"]],
            "model": model_name, "loss_fn": loss_name, "batch": batch}
+    if loss_impl == "fused" and arm == "ours":
+        res["loss_impl"] = "fused"
+        res["fused_loss_calls"] = fused_calls[0]
     if "torch_scatter" in sys.modules:  # where PointSea's scatter came from: the stub (no file) or a package
         res["torch_scatter"] = getattr(sys.modules["torch_scatter"], "__file__", None) or "stub"
     if rank == 0:
@@ -205,11 +226,13 @@ def c4_arm(arm, iters, knn, batch=32, model_name="svdformer", loss_name="get_los
 def c4(args):
     arms = ["ours", "ref"] if args.arm == "both" else [args.arm]
     if args.arm != "both":
-        return c4_arm(args.arm, args.iters, args.knn, args.batch, args.model, args.loss, args.torch_scatter)
+        return c4_arm(args.arm, args.iters, args.knn, args.batch, args.model, args.loss, args.torch_scatter,
+                      args.loss_impl)
     lines = []
     for arm, knn in (("ours", "torch"), ("ours", "ours"), ("ours", "all"), ("ref", "torch")):
         p = subprocess.run([sys.executable, __file__, "c4", "--arm", arm, "--iters", str(args.iters), "--knn", knn, "--batch", str(args.batch),
-                            "--model", args.model, "--loss", args.loss, "--torch-scatter", args.torch_scatter],
+                            "--model", args.model, "--loss", args.loss, "--torch-scatter", args.torch_scatter,
+                            "--loss-impl", args.loss_impl],
                            capture_output=True, text=True)
         last = [ln for ln in p.stdout.strip().splitlines() if ln.startswith("{")]
         if not last:
@@ -285,5 +308,7 @@ if __name__ == "__main__":
     ap.add_argument("--loss", default="get_loss", choices=["get_loss", "get_loss_PM"])
     ap.add_argument("--torch-scatter", default="stub", choices=["stub", "dropin"],
                     help="c4 pointsea: arm ours imports torch_scatter from the drop-in instead of the stand-in")
+    ap.add_argument("--loss-impl", default="composed", choices=["composed", "fused"],
+                    help="c4: arm ours runs utils/loss_utils' Chamfer losses on the fused ops (patch_loss_utils training=True)")
     a = ap.parse_args()
     {"c4": c4, "c5": c5}[a.config](a)
