@@ -216,6 +216,27 @@ int ps_fps_sample(const float* xyz, int* idx, float* new_xyz, int B, int N, int 
 int ps_fps_sample_ex(const float* xyz, int* idx, float* new_xyz, int B, int N, int npoint, int flags, int dev,
                      void* stream);
 
+/* ps_fps_sample on a ragged batch: cloud b is the first n_host[b] points of row b of xyz (B rows of `stride` points,
+ * row b at b*stride*3 floats).  n_host (HOST, B ints) is validated (1 <= n <= stride) before any CUDA call and uploaded
+ * with one copy.  idx (B,npoint) i32, relative to the row; new_xyz (B,npoint,3) or NULL.  Every cloud's samples are
+ * bit-identical to ps_fps_sample on that cloud alone (its own tie-break ranks, origin skip, n < npoint).  One launch
+ * whatever B; a cloud padded to more than 8192 ranks (opt_n_threads rounding) returns PS_ERR_UNSUPPORTED. */
+int ps_fps_sample_ragged(const float* xyz, const int* n_host, int* idx, float* new_xyz, int B, int stride, int npoint,
+                         int dev, void* stream);
+
+/* ---- online cropping (ShapeNet-55/34: utils/helpers.py:62-123 seprate_point_cloud) ------------------------------
+ * xyz (B,N,3) f32; centers_host (HOST, B x 3 floats) and num_crop_host (HOST, B ints, each in [0, N]) are validated
+ * before any CUDA call and uploaded with one copy.  Per cloud, the points are ordered by the fp32 value of
+ * torch.norm(center - p, p=2, dim=-1), ties by index (torch.argsort's stable order on CUDA):
+ *   crop row b (crop + b*crop_stride*3): the count nearest points, ascending;
+ *   keep row b (keep + b*keep_stride*3): the other N - count points, ascending; with pad_zeros != 0 instead all N
+ *     points in their original order, the cropped ones multiplied by 0.
+ * Equal counts with strides N-c / c give packed (B,N-c,3) / (B,c,3) tensors; strides N hold ragged rows.  One launch
+ * whatever B.  keep / crop may be NULL when all their rows are empty.  N outside 33..16384 returns
+ * PS_ERR_UNSUPPORTED. */
+int ps_crop_split(const float* xyz, const float* centers_host, const int* num_crop_host, float* keep, float* crop,
+                  int B, int N, int keep_stride, int crop_stride, int pad_zeros, int dev, void* stream);
+
 /* ---- gather / group ---------------------------------------------------------------------
  * Replaces gather_points_kernel_wrapper (sampling_gpu.cu:22-30) / _grad_ (:49-57):
  *   out[b,c,j] = features[b,c,idx[b,j]] ; features (B,C,N), idx (B,M) i32, out (B,C,M).

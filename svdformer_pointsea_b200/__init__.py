@@ -8,6 +8,7 @@ Public surface = the reference's op boundary (SURVEY.md 8b):
     EdgeConv (+ edge_features)                                (models/model_utils.py)
     calc_cd, calc_dcd, fscore                                 (utils/loss_utils.py, metrics/CD/fscore.py)
     losses.chamfer, chamfer_sqrt, chamfer_single_side, chamfer_single_side_sqrt  (utils/loss_utils.py:10-31)
+    seprate_point_cloud (+ patch_helpers)                     (utils/helpers.py:62-123, ShapeNet-55/34 cropping)
 `install_dropin()` makes `import metrics.CD.chamfer3D.dist_chamfer_3D` and
 `import pointnet2_ops.pointnet2_utils` resolve to this package so the reference's models and
 losses run unchanged, and `import torch_scatter` too where no torch_scatter is installed
@@ -27,6 +28,7 @@ from .metrics import calc_cd, calc_dcd, fscore, chamfer_metrics_raw, chamfer_met
 # `chamfer` itself stays at losses.chamfer: as a package attribute it would hide the `chamfer` submodule
 # (`import svdformer_pointsea_b200.chamfer as C` binds the attribute)
 from .losses import ChamferLossFunction, chamfer_loss, chamfer_sqrt, chamfer_single_side, chamfer_single_side_sqrt  # noqa: F401
+from .crop import seprate_point_cloud, crop_split_raw, fps_ragged_raw, patch_helpers  # noqa: F401
 from .dropin import install_dropin, DROPIN_PATH, DROPIN_FALLBACK_PATH  # noqa: F401
 
 __version__ = "0.1.0"

@@ -47,6 +47,8 @@ _SIGNATURES = {
     "ps_fps": [_P, _P, _c_int, _c_int, _c_int, _c_int, _P],
     "ps_fps_sample": [_P, _P, _P, _c_int, _c_int, _c_int, _c_int, _P],
     "ps_fps_sample_ex": [_P, _P, _P, _c_int, _c_int, _c_int, _c_int, _c_int, _P],
+    "ps_fps_sample_ragged": [_P, _P, _P, _P, _c_int, _c_int, _c_int, _c_int, _P],
+    "ps_crop_split": [_P] * 5 + [_c_int] * 6 + [_P],
     "ps_gather_fwd": [_P, _P, _P, _c_int, _c_int, _c_int, _c_int, _c_int, _P],
     "ps_gather_bwd": [_P, _P, _P, _c_int, _c_int, _c_int, _c_int, _c_int, _P],
     "ps_group_fwd": [_P, _P, _P, _c_int, _c_int, _c_int, _c_int, _c_int, _c_int, _P],

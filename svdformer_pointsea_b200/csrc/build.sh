@@ -6,7 +6,7 @@ OUT="$HERE/../lib"
 mkdir -p "$OUT"
 NVCC="${NVCC:-/usr/local/cuda/bin/nvcc}"
 FLAGS=(-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC -Xptxas -v)
-SRCS=(runtime.cu comm.cu step.cu chamfer.cu chamfer_sym.cu fps.cu gather_group.cu neighbors.cu knn_select.cu host_pipeline.cu feature_knn.cu metrics.cu scatter.cu chamfer_loss.cu)
+SRCS=(runtime.cu comm.cu step.cu chamfer.cu chamfer_sym.cu fps.cu gather_group.cu neighbors.cu knn_select.cu host_pipeline.cu feature_knn.cu metrics.cu scatter.cu chamfer_loss.cu crop.cu)
 OBJS=()
 pids=()
 for s in "${SRCS[@]}"; do

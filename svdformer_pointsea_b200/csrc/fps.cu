@@ -71,6 +71,10 @@ struct FpsArgs {
   int L;     // log2(bs) of the reference launch
   int nper;  // ceil(N / bs)
   const int* run_flag = nullptr;  // optional (B): a cloud whose flag is 0 has been sampled by fps_pruned_kernel already
+  // ragged batches (fps_small_kernel<..., true>): cloud b is the first part[b].x points of row b (rows of `stride`
+  // points), with its own log2(bs) = part[b].y and nper = part[b].z
+  const int4* part = nullptr;
+  long long stride = 0;
 };
 
 // rank -> point index (may be >= N for the padding ranks of the last rows)
@@ -564,7 +568,7 @@ static int dispatch_lean(int PP, const FpsArgs& a, int B, int C, cudaStream_t s)
 // looked up in the CTA's own shared-memory copy of the cloud by its rank, as fps_pruned_kernel does: two REDUX, one
 // store, one barrier, one load, two REDUX, three broadcast loads.  Same dealing of points to threads in rank order,
 // same selection (distance desc, rank asc), same -1 convention for skipped / padding points as fps_kernel.
-template <int PP, int T>
+template <int PP, int T, bool RAGGED = false>
 __global__ void __launch_bounds__(T, 1) fps_small_kernel(const FpsArgs a) {
   constexpr int P = 2 * PP;
   constexpr int WARPS = T / 32;
@@ -575,12 +579,17 @@ __global__ void __launch_bounds__(T, 1) fps_small_kernel(const FpsArgs a) {
   __shared__ int2 slots[2][WARPS];
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   if (a.run_flag && __ldg(a.run_flag + b) == 0) return;
-  const int N = a.N;
+  int N = a.N, L = a.L, nper = a.nper;
   const float* cloud = a.xyz + (size_t)b * N * 3;
+  if constexpr (RAGGED) {
+    const int4 pt = a.part[b];
+    N = pt.x; L = pt.y; nper = pt.z;
+    cloud = a.xyz + (size_t)b * a.stride * 3;
+  }
   int* out = a.idx + (size_t)b * a.npoint;
   float* oxyz = a.new_xyz ? a.new_xyz + (size_t)b * a.npoint * 3 : nullptr;
   const unsigned rank0 = (unsigned)tid * P;  // this thread owns ranks [rank0, rank0 + P)
-  const unsigned R = (unsigned)a.nper << a.L;
+  const unsigned R = (unsigned)nper << L;
 
   u64 x2[PP], y2[PP], z2[PP];
   float t[P];
@@ -589,7 +598,7 @@ __global__ void __launch_bounds__(T, 1) fps_small_kernel(const FpsArgs a) {
     float xv = 0.f, yv = 0.f, zv = 0.f;
     t[i] = -1.0f;
     if (rank0 + i < R) {
-      const int k = fps_rank_to_k(rank0 + i, a.L, a.nper);
+      const int k = fps_rank_to_k(rank0 + i, L, nper);
       if (k < N) {
         xv = __ldg(cloud + (size_t)k * 3 + 0);
         yv = __ldg(cloud + (size_t)k * 3 + 1);
@@ -651,7 +660,7 @@ __global__ void __launch_bounds__(T, 1) fps_small_kernel(const FpsArgs a) {
     int k = 0;
     float ox = p0x, oy = p0y, oz = p0z;
     if (j && gk != 0xffffffffu) {
-      k = fps_rank_to_k(gk, a.L, a.nper);
+      k = fps_rank_to_k(gk, L, nper);
       const unsigned wt = gk / (unsigned)P, wi = gk % (unsigned)P;
       ox = px[wi * T + wt]; oy = py[wi * T + wt]; oz = pz[wi * T + wt];
     }
@@ -660,10 +669,10 @@ __global__ void __launch_bounds__(T, 1) fps_small_kernel(const FpsArgs a) {
   }
 }
 
-template <int PP, int T>
+template <int PP, int T, bool RAGGED = false>
 static int launch_fps_small(const FpsArgs& a, int B, cudaStream_t stream) {
   const size_t smem = (size_t)3 * 2 * PP * T * sizeof(float);
-  auto kern = fps_small_kernel<PP, T>;
+  auto kern = fps_small_kernel<PP, T, RAGGED>;
   if (smem + 1024 > 48 * 1024) PS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));  // + static slots
   kern<<<B, T, smem, stream>>>(a);
   PS_LAUNCH_CHECK();
@@ -1229,4 +1238,54 @@ extern "C" int ps_fps_sample_ex(const float* xyz, int* idx, float* new_xyz, int 
   if (pl.C == 1) return dispatch_pp<256, 0>(pl.PP, a, B, pl.C, stream);
   if (pl.C <= 4) return poll ? dispatch_pp<256, 3>(pl.PP, a, B, pl.C, stream) : dispatch_pp<256, 1>(pl.PP, a, B, pl.C, stream);
   return dispatch_pp<256, 2>(pl.PP, a, B, pl.C, stream);
+}
+
+// Ragged batch: cloud b is the first n_host[b] points of row b, sampled exactly as ps_fps_sample samples that cloud on
+// its own (its own bs = opt_n_threads(n) and nper, hence its own tie-break ranks).  One launch of the single-CTA kernel
+// for the whole batch, sized by its largest cloud; a smaller cloud leaves the ranks beyond its own as padding.
+extern "C" int ps_fps_sample_ragged(const float* xyz, const int* n_host, int* idx, float* new_xyz, int B, int stride,
+                                    int npoint, int dev, void* stream_) {
+  PS_REQUIRE(B >= 0 && stride >= 0 && npoint >= 0, "ps_fps_sample_ragged: bad sizes B=%d stride=%d npoint=%d", B, stride,
+             npoint);
+  if (B == 0 || npoint == 0) return PS_OK;
+  PS_REQUIRE(xyz && n_host && idx, "ps_fps_sample_ragged: null pointer");
+  long long Rmax = 0;
+  for (int b = 0; b < B; b++) {
+    const int n = n_host[b];
+    PS_REQUIRE(n >= 1 && n <= stride, "ps_fps_sample_ragged: size %d of cloud %d outside [1, stride=%d]", n, b, stride);
+    const int L = ref_block_log2(n);
+    const long long R = (long long)ceil_div(n, 1 << L) << L;
+    if (R > Rmax) Rmax = R;
+  }
+  if (Rmax > 8192)
+    return set_error(PS_ERR_UNSUPPORTED, "ps_fps_sample_ragged: a cloud of %lld padded points exceeds the 8192 one CTA holds",
+                     Rmax);
+  DeviceGuard guard(dev);
+  if (!guard.ok) return set_error(PS_ERR_CUDA, "ps_fps_sample_ragged: cannot select device %d", dev);
+  cudaStream_t stream = (cudaStream_t)stream_;
+  int4* host_part = new int4[B];
+  for (int b = 0; b < B; b++) {
+    const int L = ref_block_log2(n_host[b]);
+    host_part[b] = make_int4(n_host[b], L, ceil_div(n_host[b], 1 << L), 0);
+  }
+  ScratchGuard part;
+  int rc = part.alloc((size_t)B * sizeof(int4), dev, stream);
+  // pageable source: the copy has taken the bytes when it returns, so the staging array can go at once
+  if (rc == PS_OK && cudaMemcpyAsync(part.ptr, host_part, (size_t)B * sizeof(int4), cudaMemcpyHostToDevice, stream) !=
+                         cudaSuccess)
+    rc = set_error(PS_ERR_CUDA, "ps_fps_sample_ragged: upload of the cloud sizes failed: %s",
+                   cudaGetErrorString(cudaGetLastError()));
+  delete[] host_part;
+  if (rc) return rc;
+  FpsArgs a;
+  a.xyz = xyz; a.idx = idx; a.new_xyz = new_xyz; a.N = 0; a.npoint = npoint; a.L = 0; a.nper = 0;
+  a.part = static_cast<const int4*>(part.ptr);
+  a.stride = stride;
+  if (Rmax <= 512) rc = launch_fps_small<2, 128, true>(a, B, stream);
+  else if (Rmax <= 1024) rc = launch_fps_small<4, 128, true>(a, B, stream);
+  else if (Rmax <= 2048) rc = launch_fps_small<4, 256, true>(a, B, stream);
+  else if (Rmax <= 4096) rc = launch_fps_small<4, 512, true>(a, B, stream);
+  else rc = launch_fps_small<8, 512, true>(a, B, stream);
+  if (rc) return rc;
+  return part.release();
 }
